@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (torchrun launches N ranks for N > 1)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR     (+ what the last timed step decoded, as .npy)
 
 A "step" = one pass of the whole hot path over one batch of synthetic 16 kHz utterances:
 fbank -> ConformerEncoder -> CTC log-softmax/top-k -> ctc_prefix_beam_search -> attention_rescoring,
@@ -68,6 +69,50 @@ def _edit_distance(a, b):
             cur.append(min(prev[j] + 1, cur[j - 1] + 1, prev[j - 1] + (x != y)))
         prev = cur
     return prev[-1]
+
+
+def _padded(rows):
+    """ragged rows -> (len(rows), longest) float64 padded with -1, and the row lengths"""
+    a = np.full((len(rows), max([len(r) for r in rows] + [0])), -1.0)
+    for i, r in enumerate(rows):
+        a[i, :len(r)] = r
+    return a, np.array([len(r) for r in rows], dtype=np.float64)
+
+
+def decode_arrays(results):
+    """What decode() hands its caller for one batch, as float64 arrays (token ids and frame indices are exact): per
+    utterance the best hypothesis (tokens, times, per-token confidence: rows padded with -1, lengths in <name>_lengths),
+    its score and confidence, and the n-best lists flattened over hypotheses in utterance order (nbest_count per
+    utterance).  Fields a decoding mode leaves empty are omitted."""
+    out = {"score": np.array([r.score for r in results], dtype=np.float64),
+           "confidence": np.array([r.confidence for r in results], dtype=np.float64)}
+    for name in ("tokens", "times", "tokens_confidence"):
+        rows = [getattr(r, name) for r in results]
+        if all(x is not None for x in rows):
+            out[name], out[name + "_lengths"] = _padded(rows)
+    if all(r.nbest is not None for r in results):
+        out["nbest_count"] = np.array([len(r.nbest) for r in results], dtype=np.float64)
+        out["nbest"], out["nbest_lengths"] = _padded([h for r in results for h in r.nbest])
+        out["nbest_times"], _ = _padded([t for r in results for t in r.nbest_times])
+        out["nbest_scores"] = np.array([s for r in results for s in r.nbest_scores], dtype=np.float64)
+    return out
+
+
+def dump_outputs(results, out_dir, limit=64 << 20):
+    """DIR/<name>.npy for every array of decode_arrays(results), at most `limit` bytes in all: a larger batch is
+    replaced by a fixed, seeded sample of its utterances (their batch indices in utterance.npy)."""
+    idx = np.arange(len(results))
+    arrays = decode_arrays(results)
+    while sum(a.nbytes for a in arrays.values()) > limit and len(idx) > 1:
+        keep = len(idx) // 2
+        idx = np.sort(np.random.default_rng(0).choice(len(results), keep, replace=False))
+        arrays = decode_arrays([results[i] for i in idx])
+    arrays["utterance"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    print("bench.py: %d arrays (%d utterances, %d bytes) written to %s"
+          % (len(arrays), len(idx), sum(a.nbytes for a in arrays.values()), out_dir), file=sys.stderr)
 
 
 def load_peaks():
@@ -335,7 +380,11 @@ def main():
     ap.add_argument("--inflight", type=int, default=4,
                     help="batches in flight per GPU (host threads x CUDA streams sharing one weight replica); "
                          "1 = strictly sequential steps")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the decode results of the last timed step to DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
     # stdout carries exactly ONE line, the JSON result: everything else that lands on fd 1 while the benchmark runs
     # (NCCL prints its version banner there from native code) is sent to stderr instead
     sys.stdout.flush()
@@ -474,7 +523,14 @@ def main():
     sampler = ClockSampler(local)
     sampler.start()
     launches0 = lib.wb_launch_count()
-    ms = timed(lambda i, mdl: step(dev_pcm[i % NROT], mdl), args.steps)
+    last = {}
+
+    def timed_step(i, mdl):
+        res = step(dev_pcm[i % NROT], mdl)
+        if i == args.steps - 1:
+            last["res"] = res
+
+    ms = timed(timed_step, args.steps)
     launches = lib.wb_launch_count() - launches0
 
     # ---- per-kernel pass (roofline / kernel table): CUDA events around every launch, ONE batch in flight so that the
@@ -785,6 +841,8 @@ def main():
         line["cpu_baseline"] = {"value": audio / dt, "unit": "audio-s/s", "cores": host_cores(),
                                 "threads_used": arm.procs * arm.threads, "kind": arm.kind, "sample": arm.describe()}
         arm.close()
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(last["res"][args.mode], args.dump_outputs)
     if rank == 0:
         args.emit(line)
     if world > 1:

@@ -6,6 +6,7 @@ The fixtures hold OUTPUTS only (inputs and weights are regenerated from seeds at
 stay small.  TEST INFRASTRUCTURE — nothing in wenet_b200/ imports this.
 """
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -266,10 +267,194 @@ def whisper_goldens(name="whisper_tiny", recipe="whisper_tiny", ns=(32000 + 77, 
           "size %.0f KB" % (os.path.getsize(path) / 1024))
 
 
+def _ref_exe(name):
+    """oracle/_ref/<name>, built from the reference's C++ sources by oracle/Makefile"""
+    r = subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "REF=" + shim.REFERENCE_ROOT], capture_output=True,
+                       text=True)
+    assert r.returncode == 0, r.stdout + r.stderr
+    return os.path.join(ROOT, "oracle", "_ref", name)
+
+
+def _run(exe, *args, stdin=None):
+    r = subprocess.run([exe] + [str(a) for a in args], input=stdin, capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr
+    return r.stdout
+
+
+def _cxx_search(blocks):
+    """the reference's C++ CtcPrefixBeamSearch (oracle/cxx/ctc_search_ref_main.cc) on a list of (logp [T, V], beam):
+    per block the n-best as [score, tokens, times]"""
+    text = ""
+    for lp, beam in blocks:
+        text += "%d %d %d\n" % (lp.shape[0], lp.shape[1], beam)
+        text += "\n".join(" ".join("%.9g" % x for x in row) for row in lp.tolist()) + "\n"
+    lines, out, i = _run(_ref_exe("ctc_search_ref"), stdin=text).splitlines(), [], 0
+    for _ in blocks:
+        n = int(lines[i])
+        i += 1
+        hyps = []
+        for _k in range(n):
+            a, b, c = lines[i].split("|")
+            i += 1
+            hyps.append([float(a.split()[0]), [int(x) for x in b.split()], [int(x) for x in c.split()]])
+        out.append(hyps)
+    return out
+
+
+def _search_json(res):
+    return [dict(nbest=[list(x) for x in r.nbest], nbest_scores=list(r.nbest_scores), nbest_times=[list(x) for x in r.nbest_times])
+            for r in res]
+
+
+def pin_goldens(name="oracle_pin"):
+    """What tests/test_oracle_pin.py (and two checks in test_cpu.py / test_ops_gpu.py) compare the oracle with: the
+    reference's outputs - its Python modules, and its C++ front-end / CTC prefix beam search compiled into oracle/_ref -
+    on the inputs that test module builds from seeds.  Ragged results are stored as JSON strings."""
+    import json
+    import tempfile
+    import types
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import test_oracle_pin as T
+    from oracle import wenet_oracle as O
+    js = lambda x: np.array(json.dumps(x))     # noqa: E731
+    out = {}
+    # C++ front-end: slaney filterbank and mel scale, Kaldi and Whisper fbank of 2 s of noise
+    fb = _ref_exe("fbank_ref")
+    for bins in (128, 80):
+        W = np.zeros((bins, 256), dtype=np.float32)
+        for line in _run(fb, "filters", "slaney", bins, 16000, 400, 0).splitlines():
+            p = line.split()
+            b, first, n = int(p[0]), int(p[1]), int(p[2])
+            W[b, first:first + n] = [float(x) for x in p[3:3 + n]]
+        out["slaney_filters%d" % bins] = W
+    out["slaney_melscale"] = np.array([[float(f)] + [float(x) for x in line.split()[1:]] for f, line in
+                                       zip(T.MELSCALE_HZ, _run(fb, "melscale", "slaney", *T.MELSCALE_HZ).splitlines())])
+    with tempfile.TemporaryDirectory() as td:
+        path = os.path.join(td, "pcm.f32")
+        with open(path, "wb") as f:
+            f.write(T.noise_2s().numpy().astype("<f4").tobytes())
+        for key, conf, bins in (("fbank_kaldi80", "kaldi", 80), ("fbank_whisper128", "whisper", 128)):
+            out[key] = np.array([[float(x) for x in l.split()] for l in _run(fb, "fbank", conf, bins, path).splitlines()],
+                                dtype=np.float32)
+    # C++ and Python CTC prefix beam search: the known-answer test and the 40 random posterior matrices
+    out["cxx_search_kat"] = js(_cxx_search([(torch.tensor(T.KAT_PROBS).log(), 3)])[0])
+    shim.install()
+    from wenet.models.transformer.search import (DecodeResult, attention_beam_search, attention_rescoring,
+                                                 ctc_greedy_search, ctc_prefix_beam_search)
+    blocks, py = [], []
+    for lp, lens, beam in T.random_posteriors():
+        blocks += [(lp[b, :int(lens[b])], beam) for b in range(lp.shape[0])]
+        s = _search_json(ctc_prefix_beam_search(lp, lens, beam))
+        py.append(dict(nbest=[r["nbest"] for r in s], nbest_scores=[r["nbest_scores"] for r in s],
+                       nbest_times=[r["nbest_times"] for r in s], greedy=[r.tokens for r in ctc_greedy_search(lp, lens)]))
+    out["cxx_search_random"] = js(_cxx_search(blocks))
+    out["py_search_random"] = js(py)
+
+    def model_of(cfg, sd):
+        model = shim.init_reference_model(dict(cfg))
+        missing, unexpected = model.load_state_dict(sd, strict=False)
+        assert not unexpected and all(k.endswith("num_batches_tracked") for k in missing), (missing, unexpected)
+        return model.eval()
+
+    # encoder / CTC / searches / rescoring / streaming of the two tiny Conformer variants
+    for variant in ("u2pp", "nonstream_bn"):
+        cfg, p = T.pin_model(variant)
+        model = model_of(cfg, p)
+        assert model.sos_symbol() == model.eos_symbol() == cfg["output_dim"] - 1
+        k = "match_%s_" % variant
+        xs, lens = T.randn(777, 2, 131, 80), torch.tensor([131, 90])
+        with torch.no_grad():
+            enc, mask = model.encoder(xs, lens, decoding_chunk_size=-1, num_decoding_left_chunks=-1)
+            out[k + "enc_out"], out[k + "enc_mask"] = enc.numpy(), mask.numpy()
+            if variant == "u2pp":
+                out[k + "enc_out_chunk4_left2"] = model.encoder(xs, lens, decoding_chunk_size=4, num_decoding_left_chunks=2)[0].numpy()
+                att = cnn = torch.zeros(0, 0, 0, 0)
+                off = 0
+                for j, s in enumerate(T.STREAM_STARTS):
+                    y, att, cnn = model.encoder.forward_chunk(xs[0:1, s:s + 19], off, 8, att, cnn)
+                    off += y.size(1)
+                    out[k + "stream_y%d" % j], out[k + "stream_att%d" % j], out[k + "stream_cnn%d" % j] = \
+                        y.numpy(), att.numpy(), cnn.numpy()
+            lp = model.ctc_logprobs(enc)
+            out[k + "ctc_logp"] = lp.numpy()
+            el = mask.squeeze(1).sum(1)
+            out[k + "greedy"] = js([r.tokens for r in ctc_greedy_search(lp, el)])
+            rb = ctc_prefix_beam_search(lp, el, 4)
+            out[k + "beam"] = js(_search_json(rb))
+            rs = attention_rescoring(model, rb, enc, el, 0.5, 0.3 if variant == "u2pp" else 0.0)
+            out[k + "rescoring"] = js([[list(r.tokens), float(r.score)] for r in rs])
+    cfg, p = T.pin_model("u2pp")
+    model = model_of(cfg, p)
+    for chunk, left in T.CHUNK_SETTINGS:
+        k = "chunk%d_left%d_" % (chunk, left)
+        xs, lens = T.randn(777, 2, 99, 80), torch.tensor([99, 58])
+        with torch.no_grad():
+            r, rm = model.encoder(xs, lens, decoding_chunk_size=chunk, num_decoding_left_chunks=left)
+            out[k + "enc_out"], out[k + "enc_mask"] = r.numpy(), rm.numpy()
+            out[k + "stream"] = model.encoder.forward_chunk_by_chunk(xs[:1], chunk, left)[0].numpy()
+    enc, lens = T.randn(3, 3, 17, 128), torch.tensor([17, 9, 4])
+    for cw, rw in T.RESCORING_WEIGHTS:
+        ref_in = [DecodeResult(tokens=n[0], nbest=[tuple(h) for h in n], nbest_scores=sc, nbest_times=[[0] * len(h) for h in n])
+                  for n, sc in zip(T.RESCORING_NBEST, T.RESCORING_SCORES)]
+        with torch.no_grad():
+            rs = attention_rescoring(model, ref_in, enc, lens, cw, rw)
+        out["rescoring_ctc%g_rev%g" % (cw, rw)] = js([[list(r.tokens), float(r.score)] for r in rs])
+    # context biasing: the reference's ContextGraph, flattened, and its biased search
+    from wenet.utils.context_graph import ContextGraph
+    from wenet_b200 import context as CX
+    with tempfile.TemporaryDirectory() as td:
+        f = os.path.join(td, "ctx.txt")
+        with open(f, "w") as fh:
+            fh.write("\n".join(T.CONTEXT_WORDS) + "\n")
+        cg = ContextGraph(f, T.context_symbols(), None, 3.0)
+    arr = CX.flatten(cg)
+    for n in T.CONTEXT_FIELDS:
+        out["context_" + n] = np.asarray(getattr(arr, n))
+    lp, lens = T.context_posteriors()
+    out["context_search"] = js(_search_json(ctc_prefix_beam_search(lp, lens, 6, cg, 0)))
+    # decode mode "attention" of the tiny U2++ recipe
+    cfg = synth.recipe("tiny")
+    sd = synth.synth_state_dict(cfg, seed=SEED)
+    model = model_of(dict(cfg, cmvn=None), {k: v for k, v in sd.items() if not k.startswith("encoder.global_cmvn")})
+    enc, lens = T.randn(5, 2, 21, 128), torch.tensor([21, 13])
+    mask = ~O.make_pad_mask(lens, 21).unsqueeze(1)
+    with torch.no_grad():
+        out["attention_conformer"] = js([[list(r.tokens) for r in attention_beam_search(model, enc, mask, beam, lpen)]
+                                         for beam, lpen in T.ATTENTION_SETTINGS])
+    # Whisper: log-mel (restated slaney filterbank injected as librosa.filters.mel), encoder, attention decoding
+    cfg = synth.recipe("whisper_tiny")
+    model = shim.init_reference_model(dict(cfg))
+    model.load_state_dict(synth.synth_state_dict(cfg, seed=SEED), strict=True)
+    model.eval()
+    assert model.eos == cfg["tokenizer_conf"]["special_tokens"]["eot"]
+    import wenet.dataset.processor as processor
+    sys.modules["librosa"].filters = types.SimpleNamespace(
+        mel=lambda sr, n_fft, n_mels: O.slaney_mel_filters(sr, n_fft, n_mels).numpy())
+    pcm, batches = T.whisper_pin_inputs()
+    out["whisper_logmel"] = processor.compute_log_mel_spectrogram(dict(key="k", wav=pcm.unsqueeze(0), sample_rate=16000),
+                                                                  n_fft=400, hop_length=160, num_mel_bins=32)["feat"].numpy()
+    with torch.no_grad():
+        for (Tn, _), (xs, xl) in zip(T.WHISPER_LENS, batches):
+            r_out, r_mask = model.encoder(xs, xl)
+            out["whisper_enc_out%d" % Tn], out["whisper_enc_mask%d" % Tn] = r_out.numpy(), r_mask.numpy()
+        out["whisper_attention"] = js([[list(r.tokens) for r in attention_beam_search(model, r_out, r_mask, beam, lpen, T.WHISPER_INFOS)]
+                                       for beam, lpen in T.WHISPER_SETTINGS])
+    # the reference's forced Whisper prefix (add_whisper_tokens) for tests/test_cpu.py
+    from wenet.utils.common import add_whisper_tokens
+    ys_in, _ = add_whisper_tokens(cfg["tokenizer_conf"]["special_tokens"], torch.ones(2, 0, dtype=torch.long), -1,
+                                  tasks=["transcribe", "translate"], no_timestamp=True, langs=["zh", "en"], use_prev=False)
+    out["whisper_prefix"] = ys_in.numpy()
+    path = os.path.join(GOLD, name + ".npz")
+    np.savez_compressed(path, **out)
+    print(name, len(out), "arrays, size %.0f KB" % (os.path.getsize(path) / 1024))
+
+
 if __name__ == "__main__":
     os.makedirs(GOLD, exist_ok=True)
     which = sys.argv[1:] or ["fbank", "tiny", "tiny_bn", "u2pp_small", "u2pp_small_long", "u2pp_large_10s",
-                             "u2pp_small_stream", "tiny_attention", "whisper_tiny"]
+                             "u2pp_small_stream", "tiny_attention", "whisper_tiny", "oracle_pin"]
+    if "oracle_pin" in which:
+        pin_goldens()
     if "fbank" in which:
         fbank_goldens()
     if "tiny" in which:

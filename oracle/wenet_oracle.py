@@ -710,9 +710,11 @@ def beam_step(top_k_logp, top_k_index, scores, end_flag, hyps, beam_size: int, e
 
 
 def attention_beam_search(p, pre, n_layers, heads, encoder_out, encoder_mask, beam_size: int, prefix, eos: int,
-                          length_penalty: float = 0.0, flavor: str = "wenet", quant=None, maxlen: Optional[int] = None) -> List[List[int]]:
+                          length_penalty: float = 0.0, flavor: str = "wenet", quant=None, maxlen: Optional[int] = None,
+                          return_beams: bool = False):
     """search.py:252-371.  prefix: (B, P) long - [[sos]] * B for wenet models, add_whisper_tokens' forced start for
-    Whisper (common.py:198-226).  Returns the best hypothesis of every utterance (prefix and eos stripped)."""
+    Whisper (common.py:198-226).  Returns the best hypothesis of every utterance (prefix and eos stripped); with
+    return_beams also every utterance's final beams as (hypothesis, score) pairs."""
     B = encoder_out.shape[0]
     if maxlen is None:
         maxlen = encoder_out.shape[1]      # the reference's bound (search.py:263); tests may shorten the loop
@@ -731,8 +733,8 @@ def attention_beam_search(p, pre, n_layers, heads, encoder_out, encoder_mask, be
     lengths = hyps.ne(eos).sum(dim=1).view(B, beam_size).float()
     scores = scores / lengths.pow(length_penalty)
     best = scores.argmax(dim=-1)
-    out = []
-    for b in range(B):
-        h = hyps[b * beam_size + int(best[b])][P:]
-        out.append(h[h != eos].tolist())
+    strip = lambda h: h[P:][h[P:] != eos].tolist()      # noqa: E731
+    out = [strip(hyps[b * beam_size + int(best[b])]) for b in range(B)]
+    if return_beams:
+        return out, [[(strip(hyps[b * beam_size + n]), float(scores[b, n])) for n in range(beam_size)] for b in range(B)]
     return out

@@ -1,83 +1,91 @@
-"""Pin the CPU oracle (oracle/wenet_oracle.py) against the REAL reference where it is available
-(build container) and against the reference's own known-answer test everywhere."""
+"""Pin the CPU oracle (oracle/wenet_oracle.py) against the reference: its Python modules and its C++ front-end and CTC
+prefix beam search.  What the reference computed on the inputs below is stored in tests/golden/oracle_pin.npz
+(oracle/make_goldens.py regenerates it from a reference tree, using the input functions of this module); the tests
+recompute the oracle side and compare.  The reference's own known-answer test is checked everywhere."""
+import json
 import math
-import os
-import sys
 
 import pytest
 import torch
 
+from helpers import load_golden
 from oracle import shim
 from oracle import wenet_oracle as O
+from wenet_b200 import synth
 
-needs_ref = pytest.mark.skipif(not shim.have_reference(), reason="/root/reference not present (GPU box)")
+needs_ref = pytest.mark.skipif(not shim.have_reference(), reason="needs a reference tree (WENET_REFERENCE_ROOT)")
 
-
-def _fbank_ref():
-    """oracle/_ref/fbank_ref: the reference's C++ front-end (runtime/core/frontend/fbank.h + fft.cc) behind the driver
-    oracle/cxx/fbank_ref_main.cc; built here when /root/reference is present, prebuilt on the GPU box."""
-    import subprocess
-    exe = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "fbank_ref")
-    if os.path.isdir("/root/reference/runtime/core/frontend"):
-        r = subprocess.run(["make", "-C", os.path.dirname(os.path.dirname(exe))], capture_output=True, text=True)
-        assert r.returncode == 0, r.stdout + r.stderr
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/fbank_ref not built (no /root/reference here)")
-
-    def run(*args):
-        r = subprocess.run([exe] + [str(a) for a in args], capture_output=True, text=True, timeout=120)
-        assert r.returncode == 0, r.stderr
-        return r.stdout
-    return run
+MELSCALE_HZ = [0.0, 20.0, 333.3, 999.9, 1000.0, 1000.1, 2500.0, 7999.0, 8000.0]
+_G = {}
 
 
-def _ref_filters(run, mel, bins, low):
-    W = torch.zeros(bins, 256)
-    for line in run("filters", mel, bins, 16000, 400, low).splitlines():
-        p = line.split()
-        b, first, n = int(p[0]), int(p[1]), int(p[2])
-        W[b, first:first + n] = torch.tensor([float(x) for x in p[3:3 + n]])
-    return W
+def gold(key):
+    """the reference's output stored under `key`; ragged results are JSON strings"""
+    if not _G:
+        _G.update(load_golden("oracle_pin"))
+    v = _G[key]
+    return json.loads(str(v)) if v.dtype.kind == "U" else torch.from_numpy(v.copy())
+
+
+def noise_2s():
+    """2 s + 123 samples of int16-range noise (the C++ front-end pins, and tests/test_ops_gpu.py)"""
+    g = torch.Generator().manual_seed(3)
+    return (torch.randn(16000 * 2 + 123, generator=g) * 3000).clamp(-32767, 32767).round()
+
+
+def random_posteriors():
+    """40 random CTC posterior matrices (peaky and flat, blank-heavy, repeated frames, beams up to the vocabulary size):
+    per case (log-probs [B, T, V], lengths [B], beam)"""
+    g = torch.Generator().manual_seed(2024)
+    cases = []
+    for case in range(40):
+        B = 1 + case % 3
+        T = int(torch.randint(1, 48, (1,), generator=g))
+        V = int(torch.randint(3, 14, (1,), generator=g))
+        beam = min(int(torch.randint(1, 8, (1,), generator=g)), V)   # the reference's topk(beam) needs beam <= V
+        logits = torch.randn(B, T, V, generator=g) * [0.5, 2.0, 6.0][case % 3]
+        logits[..., 0] += [0.0, 1.5, 3.0][(case // 3) % 3]          # blank-heavy cases
+        if case % 4 == 0:                                            # runs of the same token
+            logits = logits.repeat_interleave(2, dim=1)[:, :T]
+        lp = logits.log_softmax(-1)
+        lens = torch.randint(1, T + 1, (B,), generator=g)
+        lens[0] = T
+        cases.append((lp, lens, beam))
+    return cases
 
 
 @pytest.mark.parametrize("bins", [128, 80])
 def test_slaney_mel_filters_vs_reference_cxx(bins):
     """The slaney filterbank (the one function the Python reference takes from librosa, which is not installed): the
     oracle's restatement against the REFERENCE'S OWN C++ implementation, runtime/core/frontend/fbank.h:91-150 (InitMelFilters,
-    MelType::kSlaney) with :176-218 (MelScale / InverseMelScale), compiled from the reference sources.  The C++ front-end
-    works on a 512-point FFT grid (UpperPowerOfTwo(400)); the frequency grid is the only place n_fft enters the restatement,
-    so it is evaluated at n_fft = 512: same support, weights equal to fp32 rounding."""
-    run = _fbank_ref()
-    W = _ref_filters(run, "slaney", bins, 0)
+    MelType::kSlaney) with :176-218 (MelScale / InverseMelScale), compiled from the reference sources (oracle/Makefile).
+    The C++ front-end works on a 512-point FFT grid (UpperPowerOfTwo(400)); the frequency grid is the only place n_fft
+    enters the restatement, so it is evaluated at n_fft = 512: same support, weights equal to fp32 rounding."""
+    W = gold("slaney_filters%d" % bins)
     mine = O.slaney_mel_filters(16000, 512, bins)[:, :256]
     assert torch.equal(W > 0, mine > 0)
     assert (W - mine).abs().max().item() < 1e-5 * mine.max().item()
-    # the scale functions themselves, below and above the 1 kHz knee
-    fs = [0.0, 20.0, 333.3, 999.9, 1000.0, 1000.1, 2500.0, 7999.0, 8000.0]
+    # the scale functions themselves, below and above the 1 kHz knee: the reference's (Hz, mel, inverse) triples
     f_sp, knee, step = 200.0 / 3, 1000.0, math.log(6.4) / 27.0
-    for line, f in zip(run("melscale", "slaney", *fs).splitlines(), fs):
-        _, mel, inv = (float(x) for x in line.split())
+    ref = gold("slaney_melscale").tolist()
+    assert [r[0] for r in ref] == pytest.approx(MELSCALE_HZ, rel=1e-6)
+    for (_, mel, inv), f in zip(ref, MELSCALE_HZ):
         want = knee / f_sp + math.log(f / knee) / step if f >= knee else f / f_sp
         assert abs(mel - want) < 1e-5 * max(1.0, want) and abs(inv - f) < 1e-5 * max(1.0, f)
 
 
-def test_fbank_vs_reference_cxx(tmp_path):
-    """Kaldi fbank: the oracle (pinned to torchaudio above) against the reference's own C++ front-end in the runtime's
+def test_fbank_vs_reference_cxx():
+    """Kaldi fbank: the oracle (pinned to torchaudio below) against the reference's own C++ front-end in the runtime's
     configuration (feature_pipeline.h:55-63 -> fbank.h:247-326: povey window, HTK mel from 20 Hz, pre-emphasis, DC removal,
     natural log with an FLT_EPSILON floor) on 2 s of noise; and the C++ Whisper configuration (feature_pipeline.h:64-73:
     hanning, slaney, log10, max - 8 clamp, (x + 4) / 4) against a per-frame restatement that uses the oracle's slaney
     filterbank.  (The Python Whisper front-end frames differently - centred STFT of size 400 - and is pinned separately.)"""
-    import numpy as np
-    run = _fbank_ref()
-    g = torch.Generator().manual_seed(3)
-    wav = (torch.randn(16000 * 2 + 123, generator=g) * 3000).clamp(-32767, 32767).round()
-    path = tmp_path / "pcm.f32"
-    path.write_bytes(wav.numpy().astype("<f4").tobytes())
-    ref = torch.tensor([[float(x) for x in l.split()] for l in run("fbank", "kaldi", 80, path).splitlines()])
+    wav = noise_2s()
+    ref = gold("fbank_kaldi80")
     got = O.fbank(wav)
     assert got.shape == ref.shape
     assert (got - ref).abs().max().item() < 1e-3 and (got - ref).abs().mean().item() < 5e-5
-    refw = torch.tensor([[float(x) for x in l.split()] for l in run("fbank", "whisper", 128, path).splitlines()])
+    refw = gold("fbank_whisper128")
     m = 1 + (wav.numel() - 400) // 160
     frames = (wav / 32768.0).as_strided((m, 400), (160, 1)).clone()
     frames = frames - frames.mean(1, keepdim=True)                     # fbank.h:281-286 (remove_dc_offset stays on)
@@ -90,69 +98,28 @@ def test_fbank_vs_reference_cxx(tmp_path):
     assert refw.shape == lg.shape and (refw - lg).abs().max().item() < 1e-4
 
 
-def _ctc_search_ref(blocks):
-    """oracle/_ref/ctc_search_ref (the reference's C++ CtcPrefixBeamSearch behind oracle/cxx/ctc_search_ref_main.cc) on a list
-    of (logp [T, V], beam): per block the n-best (score, tokens, times)."""
-    import subprocess
-    exe = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "ctc_search_ref")
-    if os.path.isdir("/root/reference/runtime/core/decoder"):
-        r = subprocess.run(["make", "-C", os.path.dirname(os.path.dirname(exe))], capture_output=True, text=True)
-        assert r.returncode == 0, r.stdout + r.stderr
-    if not os.path.exists(exe):
-        pytest.skip("oracle/_ref/ctc_search_ref not built (no /root/reference here)")
-    text = ""
-    for lp, beam in blocks:
-        text += "%d %d %d\n" % (lp.shape[0], lp.shape[1], beam)
-        text += "\n".join(" ".join("%.9g" % x for x in row) for row in lp.tolist()) + "\n"
-    r = subprocess.run([exe], input=text, capture_output=True, text=True, timeout=120)
-    assert r.returncode == 0, r.stderr
-    lines, out, i = r.stdout.splitlines(), [], 0
-    for _ in blocks:
-        n = int(lines[i])
-        i += 1
-        hyps = []
-        for _k in range(n):
-            a, b, c = lines[i].split("|")
-            i += 1
-            hyps.append((float(a.split()[0]), [int(x) for x in b.split()], [int(x) for x in c.split()]))
-        out.append(hyps)
-    return out
+KAT_PROBS = [[0.25, 0.40, 0.35], [0.40, 0.35, 0.25], [0.10, 0.50, 0.40]]
 
 
 def test_reference_cxx_search_kat_and_best_path():
     """The reference has TWO implementations of the CTC prefix beam search: wenet/models/transformer/search.py:127-249 (the
     Python API this build drops in under; the oracle equals it exactly, below) and runtime/core/decoder/ctc_prefix_beam_search.cc
-    (the C++ runtime, float32, its own merge / time rules).  The C++ one is compiled from the reference sources and
+    (the C++ runtime, float32, its own merge / time rules).  The C++ one, compiled from the reference sources,
     (a) reproduces the reference's known-answer test - the vectors test_prefix_beam_search_kat holds were transcribed from
     ctc_prefix_beam_search_test.cc:29-72 - and (b) picks the same BEST hypothesis as the oracle on all utterances of the 40
     random posterior matrices.  Deeper n-best entries, scores and times differ between the reference's own two
-    implementations (measured here: full list equal on 74 of 79 utterances, best-path scores up to 0.09 apart), which is why
-    the parity target is the Python search."""
-    probs = torch.tensor([[0.25, 0.40, 0.35], [0.40, 0.35, 0.25], [0.10, 0.50, 0.40]]).log()
-    kat = _ctc_search_ref([(probs, 3)])[0]
+    implementations (full list equal on 74 of 79 utterances, best-path scores up to 0.09 apart), which is why the parity
+    target is the Python search.  Each C++ hypothesis is stored as [score, tokens, times]."""
+    kat = gold("cxx_search_kat")
     assert [h[1] for h in kat] == [[2, 1], [1, 2], [1]]
     for (score, _, _), want in zip(kat, [0.2185, 0.1550, 0.1525]):
         assert abs(math.exp(score) - want) < 1e-4
     assert [h[2] for h in kat] == [[0, 2], [0, 2], [2]]
-    g = torch.Generator().manual_seed(2024)
-    blocks, want = [], []
-    for case in range(40):
-        B = 1 + case % 3
-        T = int(torch.randint(1, 48, (1,), generator=g))
-        V = int(torch.randint(3, 14, (1,), generator=g))
-        beam = min(int(torch.randint(1, 8, (1,), generator=g)), V)
-        logits = torch.randn(B, T, V, generator=g) * [0.5, 2.0, 6.0][case % 3]
-        logits[..., 0] += [0.0, 1.5, 3.0][(case // 3) % 3]
-        if case % 4 == 0:
-            logits = logits.repeat_interleave(2, dim=1)[:, :T]
-        lp = logits.log_softmax(-1)
-        lens = torch.randint(1, T + 1, (B,), generator=g)
-        lens[0] = T
-        got = O.ctc_prefix_beam_search(lp, lens, beam)
-        for b in range(B):
-            blocks.append((lp[b, :int(lens[b])], beam))
-            want.append(got[b])
-    ref = _ctc_search_ref(blocks)
+    want = []
+    for lp, lens, beam in random_posteriors():
+        want += O.ctc_prefix_beam_search(lp, lens, beam)
+    ref = gold("cxx_search_random")
+    assert len(ref) == len(want) == 79
     same_list = 0
     for r, o in zip(ref, want):
         assert r[0][1] == o["nbest"][0]
@@ -162,7 +129,7 @@ def test_reference_cxx_search_kat_and_best_path():
 
 def test_prefix_beam_search_kat():
     """runtime/core/test/ctc_prefix_beam_search_test.cc:29-72 (the reference's only golden vector on this path)."""
-    probs = torch.tensor([[0.25, 0.40, 0.35], [0.40, 0.35, 0.25], [0.10, 0.50, 0.40]]).log().unsqueeze(0)
+    probs = torch.tensor(KAT_PROBS).log().unsqueeze(0)
     r = O.ctc_prefix_beam_search(probs, torch.tensor([3]), 3)[0]
     assert r["nbest"] == [[2, 1], [1, 2], [1]]
     for got, want in zip(r["nbest_scores"], [0.2185, 0.1550, 0.1525]):
@@ -172,33 +139,18 @@ def test_prefix_beam_search_kat():
     assert O.ctc_greedy_search(probs, torch.tensor([3])) == [[1, 1]]
 
 
-@needs_ref
 def test_prefix_beam_search_random_posteriors_vs_reference():
-    """search.py:127-249 on 40 random posterior matrices (peaky and flat, blank-heavy, repeated frames, beams up to the vocabulary size):
-    n-best token lists, fp64 scores and times of the oracle equal the reference's, element for element."""
-    shim.install()
-    from wenet.models.transformer.search import ctc_greedy_search, ctc_prefix_beam_search
-    g = torch.Generator().manual_seed(2024)
-    for case in range(40):
-        B = 1 + case % 3
-        T = int(torch.randint(1, 48, (1,), generator=g))
-        V = int(torch.randint(3, 14, (1,), generator=g))
-        beam = min(int(torch.randint(1, 8, (1,), generator=g)), V)   # the reference's topk(beam) needs beam <= V
-        sharp = [0.5, 2.0, 6.0][case % 3]
-        logits = torch.randn(B, T, V, generator=g) * sharp
-        logits[..., 0] += [0.0, 1.5, 3.0][(case // 3) % 3]          # blank-heavy cases
-        if case % 4 == 0:                                            # runs of the same token
-            logits = logits.repeat_interleave(2, dim=1)[:, :T]
-        lp = logits.log_softmax(-1)
-        lens = torch.randint(1, T + 1, (B,), generator=g)
-        lens[0] = T
-        ref = ctc_prefix_beam_search(lp, lens, beam)
+    """search.py:127-249 on the 40 random posterior matrices: n-best token lists, fp64 scores and times of the oracle equal
+    the reference's, element for element; ctc_greedy_search too."""
+    ref = gold("py_search_random")
+    for case, (lp, lens, beam) in enumerate(random_posteriors()):
         got = O.ctc_prefix_beam_search(lp, lens, beam)
-        for r, o in zip(ref, got):
-            assert [list(x) for x in r.nbest] == o["nbest"], case
-            assert r.nbest_scores == o["nbest_scores"], case
-            assert [list(x) for x in r.nbest_times] == o["nbest_times"], case
-        assert [r.tokens for r in ctc_greedy_search(lp, lens)] == O.ctc_greedy_search(lp, lens), case
+        assert len(ref[case]["nbest"]) == len(got), case
+        for b, o in enumerate(got):
+            assert ref[case]["nbest"][b] == o["nbest"], case
+            assert ref[case]["nbest_scores"][b] == o["nbest_scores"], case
+            assert ref[case]["nbest_times"][b] == o["nbest_times"], case
+        assert ref[case]["greedy"] == O.ctc_greedy_search(lp, lens), case
 
 
 def test_fbank_vs_torchaudio():
@@ -267,94 +219,93 @@ def _tiny_cfg(bidir=True, causal=True, norm="layer_norm", kernel=8):
     }
 
 
-@needs_ref
+
+
+def randn(seed, *shape):
+    return torch.randn(*shape, generator=torch.Generator().manual_seed(seed))
+
+
+def pin_model(variant):
+    """config and weights of the model pins: seeded synthetic weights (wenet_b200/synth.py, CTC head not sharpened), which
+    the reference model loads for the goldens"""
+    cfg = {"u2pp": _tiny_cfg(bidir=True),
+           "nonstream_bn": _tiny_cfg(bidir=False, causal=False, norm="batch_norm", kernel=15)}[variant]
+    return cfg, synth.synth_state_dict(cfg, seed=777, ctc_alpha=1.0)
+
+
+STREAM_STARTS = range(0, 131 - 18, 16)      # forward_chunk steps of 19 input frames (chunk 4 after subsampling)
+
+
 @pytest.mark.parametrize("variant", ["u2pp", "nonstream_bn"])
 def test_oracle_matches_reference(variant):
-    torch.manual_seed(777)
-    cfg = _tiny_cfg(bidir=True) if variant == "u2pp" else _tiny_cfg(bidir=False, causal=False, norm="batch_norm", kernel=15)
-    model = shim.init_reference_model(cfg)
-    # make BatchNorm statistics non-trivial
-    for n, b in model.named_buffers():
-        if n.endswith("running_mean"):
-            b.copy_(torch.randn_like(b) * 0.1)
-        if n.endswith("running_var"):
-            b.copy_(torch.rand_like(b) + 0.5)
-    p = {k: v.detach().clone() for k, v in model.state_dict().items()}
+    cfg, p = pin_model(variant)
     ecfg = O.encoder_cfg(p, heads=2, causal=cfg["encoder_conf"]["causal"], cnn_norm=cfg["encoder_conf"]["cnn_module_norm"])
-    xs = torch.randn(2, 131, 80)
+    xs = randn(777, 2, 131, 80)
     lens = torch.tensor([131, 90])
+    k = "match_%s_" % variant
+    ref_out, ref_mask = gold(k + "enc_out"), gold(k + "enc_mask")
     with torch.no_grad():
-        ref_out, ref_mask = model.encoder(xs, lens, decoding_chunk_size=-1, num_decoding_left_chunks=-1)
         got_out, got_mask = O.encoder_forward(p, ecfg, xs, lens)
         assert torch.equal(ref_mask, got_mask)
         for b in range(2):
             n = int(ref_mask[b].sum())
             assert (ref_out[b, :n] - got_out[b, :n]).abs().max().item() < 2e-5
         if variant == "u2pp":
-            r2, _ = model.encoder(xs, lens, decoding_chunk_size=4, num_decoding_left_chunks=2)
+            r2 = gold(k + "enc_out_chunk4_left2")
             g2, _ = O.encoder_forward(p, ecfg, xs, lens, 4, 2)
             n = int(ref_mask[1].sum())
             assert (r2[1, :n] - g2[1, :n]).abs().max().item() < 2e-5
-            # streaming chunk step (encoder.py:204-300)
-            att = torch.zeros(0, 0, 0, 0)
-            cnn = torch.zeros(0, 0, 0, 0)
-            att_o, cnn_o = att, cnn
+            # streaming chunk step (encoder.py:204-300): output and both caches after every chunk
+            att_o = cnn_o = torch.zeros(0, 0, 0, 0)
             off = 0
-            for s in range(0, 131 - 18, 16):
-                chunk_x = xs[0:1, s:s + 19]
-                y, att, cnn = model.encoder.forward_chunk(chunk_x, off, 8, att, cnn)
-                yo, att_o, cnn_o = O.encoder_forward_chunk(p, ecfg, chunk_x, off, 8, att_o, cnn_o)
+            for j, s in enumerate(STREAM_STARTS):
+                yo, att_o, cnn_o = O.encoder_forward_chunk(p, ecfg, xs[0:1, s:s + 19], off, 8, att_o, cnn_o)
+                y, att, cnn = (gold(k + "stream_%s%d" % (w, j)) for w in ("y", "att", "cnn"))
                 off += y.size(1)
                 assert (y - yo).abs().max().item() < 2e-5
                 assert (att - att_o).abs().max().item() < 2e-5 and (cnn - cnn_o).abs().max().item() < 2e-5
-        # CTC + searches
-        ref_lp = model.ctc_logprobs(ref_out)
+        # CTC + searches (the reference's searches ran on its own log-probs, as the oracle's do here)
+        ref_lp = gold(k + "ctc_logp")
         got_lp = O.ctc_logprobs(p, got_out)
         assert (ref_lp - got_lp).abs().max().item() < 5e-5
         enc_lens = ref_mask.squeeze(1).sum(1)
-        from wenet.models.transformer.search import (attention_rescoring, ctc_greedy_search,
-                                                     ctc_prefix_beam_search)
-        rg = ctc_greedy_search(ref_lp, enc_lens)
-        assert [r.tokens for r in rg] == O.ctc_greedy_search(ref_lp, enc_lens)
-        rb = ctc_prefix_beam_search(ref_lp, enc_lens, 4)
+        assert gold(k + "greedy") == O.ctc_greedy_search(ref_lp, enc_lens)
+        rb = gold(k + "beam")
         gb = O.ctc_prefix_beam_search(ref_lp, enc_lens, 4)
         for r, g in zip(rb, gb):
-            assert [list(x) for x in r.nbest] == g["nbest"]
-            assert r.nbest_scores == g["nbest_scores"]
-            assert [list(x) for x in r.nbest_times] == g["nbest_times"]
+            assert r["nbest"] == g["nbest"]
+            assert r["nbest_scores"] == g["nbest_scores"]
+            assert r["nbest_times"] == g["nbest_times"]
         rw = 0.3 if variant == "u2pp" else 0.0
-        rr = attention_rescoring(model, rb, ref_out, enc_lens, 0.5, rw)
         dcfg = dict(bidirectional=(variant == "u2pp"), layers=2, r_layers=1, heads=2)
-        gr = O.attention_rescoring(p, dcfg, gb, ref_out, enc_lens, model.sos_symbol(), model.eos_symbol(), 0.5, rw)
-        for r, g in zip(rr, gr):
-            assert list(r.tokens) == g["tokens"]
-            assert abs(r.score - g["best_score"]) < 1e-4
+        sos = eos = cfg["output_dim"] - 1
+        gr = O.attention_rescoring(p, dcfg, gb, ref_out, enc_lens, sos, eos, 0.5, rw)
+        for (tokens, score), g in zip(gold(k + "rescoring"), gr):
+            assert tokens == g["tokens"]
+            assert abs(score - g["best_score"]) < 1e-4
 
 
-@needs_ref
-@pytest.mark.parametrize("chunk,left", [(1, 0), (1, -1), (3, 1), (8, -1), (16, 4), (32, 0)])
+CHUNK_SETTINGS = [(1, 0), (1, -1), (3, 1), (8, -1), (16, 4), (32, 0)]
+
+
+@pytest.mark.parametrize("chunk,left", CHUNK_SETTINGS)
 def test_oracle_chunk_masks_and_streaming_vs_reference(chunk, left):
     """add_optional_chunk_mask (mask.py:162-227) and forward_chunk_by_chunk (encoder.py:302-362) for chunk / left-chunk
     settings from the degenerate (1 frame, no history) to wider than the utterance: the masked full forward and the chunk
     loop of the oracle equal the reference's, and (with limited history only when left >= 0) each other's cache semantics."""
-    torch.manual_seed(777)
-    cfg = _tiny_cfg(bidir=True)
-    cfg["encoder_conf"]["use_dynamic_chunk"] = True
-    cfg["encoder_conf"]["use_dynamic_left_chunk"] = False
-    model = shim.init_reference_model(cfg)
-    p = {k: v.detach().clone() for k, v in model.state_dict().items()}
+    cfg, p = pin_model("u2pp")
     ecfg = O.encoder_cfg(p, heads=2, causal=True, cnn_norm="layer_norm")
-    xs = torch.randn(2, 99, 80)
+    xs = randn(777, 2, 99, 80)
     lens = torch.tensor([99, 58])
+    k = "chunk%d_left%d_" % (chunk, left)
+    r, rm, rs = gold(k + "enc_out"), gold(k + "enc_mask"), gold(k + "stream")
     with torch.no_grad():
-        r, rm = model.encoder(xs, lens, decoding_chunk_size=chunk, num_decoding_left_chunks=left)
         o, om = O.encoder_forward(p, ecfg, xs, lens, chunk, left)
         assert torch.equal(rm, om)
         for b in range(2):
             n = int(rm[b].sum())
             assert (r[b, :n] - o[b, :n]).abs().max().item() < 2e-5, (chunk, left, b)
         # the streaming loop over one utterance (batch 1 by construction, encoder.py:330-333)
-        rs, _ = model.encoder.forward_chunk_by_chunk(xs[:1], chunk, left)
         win, stride = (chunk - 1) * 4 + 7, 4 * chunk
         att = cnn = torch.zeros(0, 0, 0, 0)
         off, outs = 0, []
@@ -370,32 +321,26 @@ def test_oracle_chunk_masks_and_streaming_vs_reference(chunk, left):
         assert (rs[0] - r[0, :rs.size(1)]).abs().max().item() < 1e-4
 
 
-@needs_ref
-@pytest.mark.parametrize("ctc_weight,reverse_weight", [(0.0, 0.0), (0.5, 0.0), (0.3, 0.3), (1.0, 0.5), (0.0, 1.0)])
+RESCORING_NBEST = [[[5, 7, 7, 30], [5, 7], [], [36]], [[2, 3, 4], [4, 3, 2]], [[11]]]
+RESCORING_SCORES = [[-1.5, -2.25, -9.0, -3.0], [-0.5, -0.5], [-0.1]]
+RESCORING_WEIGHTS = [(0.0, 0.0), (0.5, 0.0), (0.3, 0.3), (1.0, 0.5), (0.0, 1.0)]
+
+
+@pytest.mark.parametrize("ctc_weight,reverse_weight", RESCORING_WEIGHTS)
 def test_oracle_rescoring_weights_vs_reference(ctc_weight, reverse_weight):
     """attention_rescoring (search.py:374-458) over the weight settings that change which terms count: decoder only,
     CTC-weighted, bidirectional mix, right-to-left only; n-best lists with empty, single-token and equal-length hypotheses."""
-    shim.install()
-    from wenet.models.transformer.search import DecodeResult, attention_rescoring
-    torch.manual_seed(3)
-    cfg = _tiny_cfg(bidir=True)
-    model = shim.init_reference_model(cfg)
-    p = {k: v.detach().clone() for k, v in model.state_dict().items()}
-    enc = torch.randn(3, 17, 128)
+    cfg, p = pin_model("u2pp")
+    enc = randn(3, 3, 17, 128)
     lens = torch.tensor([17, 9, 4])
-    nbest = [[[5, 7, 7, 30], [5, 7], [], [36]], [[2, 3, 4], [4, 3, 2]], [[11]]]
-    scores = [[-1.5, -2.25, -9.0, -3.0], [-0.5, -0.5], [-0.1]]
-    ref_in = [DecodeResult(tokens=n[0], nbest=[tuple(h) for h in n], nbest_scores=sc, nbest_times=[[0] * len(h) for h in n])
-              for n, sc in zip(nbest, scores)]
-    got_in = [dict(nbest=n, nbest_scores=sc) for n, sc in zip(nbest, scores)]
+    got_in = [dict(nbest=n, nbest_scores=sc) for n, sc in zip(RESCORING_NBEST, RESCORING_SCORES)]
+    sos = eos = cfg["output_dim"] - 1
     with torch.no_grad():
-        ref = attention_rescoring(model, ref_in, enc, lens, ctc_weight, reverse_weight)
         dcfg = dict(bidirectional=True, layers=2, r_layers=1, heads=2)
-        got = O.attention_rescoring(p, dcfg, got_in, enc, lens, model.sos_symbol(), model.eos_symbol(), ctc_weight,
-                                    reverse_weight)
-    for r, g in zip(ref, got):
-        assert list(r.tokens) == g["tokens"]
-        assert abs(r.score - g["best_score"]) < 1e-4
+        got = O.attention_rescoring(p, dcfg, got_in, enc, lens, sos, eos, ctc_weight, reverse_weight)
+    for (tokens, score), g in zip(gold("rescoring_ctc%g_rev%g" % (ctc_weight, reverse_weight)), got):
+        assert tokens == g["tokens"]
+        assert abs(score - g["best_score"]) < 1e-4
 
 
 @needs_ref
@@ -448,115 +393,111 @@ def test_plugin_config_reconstruction_and_registry():
     assert im.WENET_MODEL_CLASSES["asr_model"] is ASRModel
 
 
-@needs_ref
-def test_context_graph_restated_vs_reference(tmp_path):
-    """Context biasing (SURVEY.md section 8f-3): wenet_b200.context.flatten / build reproduce the reference's
-    ContextGraph (context_graph.py:103-200), and the oracle's prefix beam search with the flattened graph equals the
-    reference's ctc_prefix_beam_search(..., context_graph) - prefixes, float64 scores (incl. the finalize() rule) and
-    times - while differing from the un-biased search."""
-    import numpy as np
-    shim.install()
-    from wenet.models.transformer.search import ctc_prefix_beam_search as ref_pbs
-    from wenet.utils.context_graph import ContextGraph
-    from wenet_b200 import context as CX
-    V = 30
+
+
+CONTEXT_WORDS = ["abc", "bcd", "ab", "cdeab", "xyz", "qrs q"]
+CONTEXT_FIELDS = ("child_off", "child_tok", "child_node", "fail", "token", "node_score", "token_score", "output_score")
+
+
+def context_symbols(V=30):
     sym = {"<blank>": 0, "<unk>": 1}
     for i in range(2, V):
         sym[chr(ord("a") + i - 2) if i < 28 else "z%d" % i] = i
-    words = ["abc", "bcd", "ab", "cdeab", "xyz", "qrs q"]
-    f = tmp_path / "ctx.txt"
-    f.write_text("\n".join(words) + "\n")
-    cg = ContextGraph(str(f), sym, None, 3.0)
-    arr = CX.flatten(cg)
-    arr2 = CX.build([[sym.get(c if c != " " else "▁", sym["<unk>"]) for c in w] for w in words], 3.0)
-    for n in ("child_off", "child_tok", "child_node", "fail", "token", "node_score", "token_score", "output_score"):
-        assert np.array_equal(getattr(arr, n), getattr(arr2, n)), n
-    torch.manual_seed(1)
-    T = 60
-    logits = torch.randn(3, T, V) * 2
+    return sym
+
+
+def context_posteriors(V=30, T=60):
+    logits = randn(1, 3, T, V) * 2
     logits[:, :, 0] += 2.0
-    lp = logits.log_softmax(-1)
-    lens = torch.tensor([T, 41, 7])
-    ref = ref_pbs(lp, lens, 6, cg, 0)
+    return logits.log_softmax(-1), torch.tensor([T, 41, 7])
+
+
+def test_context_graph_restated_vs_reference():
+    """Context biasing (SURVEY.md section 8f-3): wenet_b200.context.build reproduces the arrays wenet_b200.context.flatten
+    makes of the reference's ContextGraph (context_graph.py:103-200) for the same phrases, and the oracle's prefix beam
+    search with that graph equals the reference's ctc_prefix_beam_search(..., context_graph) - prefixes, float64 scores
+    (incl. the finalize() rule) and times - while differing from the un-biased search."""
+    import numpy as np
+    from wenet_b200 import context as CX
+    sym = context_symbols()
+    arr = CX.build([[sym.get(c if c != " " else "\u2581", sym["<unk>"]) for c in w] for w in CONTEXT_WORDS], 3.0)
+    for n in CONTEXT_FIELDS:
+        assert np.array_equal(getattr(arr, n), gold("context_" + n).numpy()), n
+    lp, lens = context_posteriors()
+    ref = gold("context_search")
     got = O.ctc_prefix_beam_search(lp, lens, 6, 0, arr)
     plain = O.ctc_prefix_beam_search(lp, lens, 6, 0)
     for a, b in zip(ref, got):
-        assert [list(x) for x in a.nbest] == b["nbest"]
-        assert a.nbest_scores == b["nbest_scores"]
-        assert a.nbest_times == b["nbest_times"]
+        assert a["nbest"] == b["nbest"]
+        assert a["nbest_scores"] == b["nbest_scores"]
+        assert a["nbest_times"] == b["nbest_times"]
     assert any(g["nbest"] != p["nbest"] for g, p in zip(got, plain))
 
 
-@needs_ref
+ATTENTION_SETTINGS = [(4, 0.0), (3, 0.6)]
+
+
 def test_attention_beam_search_oracle_matches_reference_conformer():
     """decode mode "attention" of a U2++ model (asr_model.py:315-318 -> search.py:252-371, left decoder,
     decoder.py:466-488): the cache-free restatement equals the reference's cached forward_one_step loop."""
-    from wenet_b200 import synth
     cfg = synth.recipe("tiny")
-    sd = synth.synth_state_dict(cfg, seed=777)
-    model = shim.init_reference_model(dict(cfg, cmvn=None))
-    model.load_state_dict({k: v for k, v in sd.items() if k in model.state_dict()}, strict=False)
-    p = {k: v.detach().clone() for k, v in model.state_dict().items()}
-    torch.manual_seed(5)
-    enc = torch.randn(2, 21, 128)
+    p = synth.synth_state_dict(cfg, seed=777)
+    enc = randn(5, 2, 21, 128)
     lens = torch.tensor([21, 13])
     mask = ~O.make_pad_mask(lens, 21).unsqueeze(1)
-    from wenet.models.transformer.search import attention_beam_search
-    for beam, lp in ((4, 0.0), (3, 0.6)):
+    sos = eos = cfg["output_dim"] - 1
+    for (beam, lp), ref in zip(ATTENTION_SETTINGS, gold("attention_conformer")):
         with torch.no_grad():
-            ref = attention_beam_search(model, enc, mask, beam, lp)
-            got = O.attention_beam_search(p, "decoder.left_decoder", 2, 2, enc, mask, beam,
-                                          [[model.sos_symbol()]] * 2, model.eos_symbol(), lp, "wenet")
-        assert [list(r.tokens) for r in ref] == got
+            got = O.attention_beam_search(p, "decoder.left_decoder", 2, 2, enc, mask, beam, [[sos]] * 2, eos, lp, "wenet")
+        assert ref == got, (beam, lp)
 
 
-@needs_ref
-def test_whisper_oracle_matches_reference():
-    """Whisper (wenet/models/whisper/whisper.py): log-mel call site, TransformerEncoder (conv1d2 / abs_pos_whisper / gelu),
-    attention_beam_search with the forced Whisper prefix."""
-    import sys as _sys
-    from wenet_b200 import synth
-    cfg = synth.recipe("whisper_tiny")
-    sd = synth.synth_state_dict(cfg, seed=777)
-    model = shim.init_reference_model(dict(cfg))
-    model.load_state_dict(sd, strict=True)
-    p = {k: v.detach().clone() for k, v in model.state_dict().items()}
-    # log-mel: the reference's own function with the restated filterbank injected as librosa.filters.mel
-    import types
-    import wenet.dataset.processor as processor
-    lib = _sys.modules["librosa"]
-    lib.filters = types.SimpleNamespace(mel=lambda sr, n_fft, n_mels: O.slaney_mel_filters(sr, n_fft, n_mels).numpy())
+WHISPER_SETTINGS = [(4, 0.0), (1, 0.0), (6, 0.8)]     # beam 1 = greedy over the beam machinery; a length penalty
+WHISPER_INFOS = {"tasks": ["transcribe", "transcribe", "translate"], "langs": ["en", "zh", "en"]}
+WHISPER_LENS = ((150, [150, 111, 64]), (151, [151, 100, 37]))       # odd and even padded lengths (subsampling.py:171)
+
+
+def whisper_pin_inputs():
+    """the Whisper pin's audio (2 s + 77 samples) and its encoder inputs, one zero-padded batch per entry of WHISPER_LENS"""
     pcm = synth.synth_pcm(1, [16000 * 2 + 77], seed=3)[0, :16000 * 2 + 77].float() / 32768.0
-    ref = processor.compute_log_mel_spectrogram(dict(key="k", wav=pcm.unsqueeze(0), sample_rate=16000), n_fft=400,
-                                                hop_length=160, num_mel_bins=32)["feat"]
+    g = torch.Generator().manual_seed(1)
+    batches = []
+    for T, lens in WHISPER_LENS:
+        xs = torch.randn(3, T, 32, generator=g) * 0.5
+        for b in range(3):
+            xs[b, lens[b]:] = 0.0
+        batches.append((xs, torch.tensor(lens)))
+    return pcm, batches
+
+
+def test_whisper_oracle_matches_reference():
+    """Whisper (wenet/models/whisper/whisper.py): log-mel call site (the reference's own function with the restated slaney
+    filterbank injected as librosa.filters.mel), TransformerEncoder (conv1d2 / abs_pos_whisper / gelu),
+    attention_beam_search with the forced Whisper prefix."""
+    from wenet_b200.whisper import whisper_prefix
+    cfg = synth.recipe("whisper_tiny")
+    p = synth.synth_state_dict(cfg, seed=777)
+    pcm, batches = whisper_pin_inputs()
+    ref = gold("whisper_logmel")
     got = O.log_mel_spectrogram(pcm, 400, 160, 32)
     assert got.shape == ref.shape and (got - ref).abs().max().item() < 1e-5
     # slaney filterbank sanity: every filter is a non-negative triangle of area ~ 1 Hz^-1 * df (slaney norm), rows overlap
     fb = O.slaney_mel_filters(16000, 400, 128)
     assert fb.shape == (128, 201) and float(fb.min()) >= 0.0 and int((fb.sum(1) > 0).sum()) == 128
     assert abs(float((fb.sum(1) * 40.0)[100:].mean()) - 1.0) < 0.05        # bin spacing 40 Hz: area normalised filters
-    # encoder, odd and even padded lengths (subsampling.py:171 mask parity)
-    torch.manual_seed(1)
-    for T, lens in ((150, [150, 111, 64]), (151, [151, 100, 37])):
-        xs = torch.randn(3, T, 32) * 0.5
-        xl = torch.tensor(lens)
-        for b in range(3):
-            xs[b, lens[b]:] = 0.0
+    for (T, lens), (xs, xl) in zip(WHISPER_LENS, batches):
+        r_out, r_mask = gold("whisper_enc_out%d" % T), gold("whisper_enc_mask%d" % T)
         with torch.no_grad():
-            r_out, r_mask = model.encoder(xs, xl)
             g_out, g_mask = O.whisper_encoder_forward(p, 2, xs, xl)
         assert torch.equal(r_mask, g_mask)
         for b in range(3):
             n = int(r_mask[b].sum())
             assert (r_out[b, :n] - g_out[b, :n]).abs().max().item() < 2e-5
-    # attention decoding
-    from wenet.models.transformer.search import attention_beam_search
-    from wenet_b200.whisper import whisper_prefix
-    infos = {"tasks": ["transcribe", "transcribe", "translate"], "langs": ["en", "zh", "en"]}
-    prefix = whisper_prefix(cfg["tokenizer_conf"]["special_tokens"], infos["tasks"], infos["langs"])
-    for beam, lp in ((4, 0.0), (1, 0.0), (6, 0.8)):      # beam 1 = greedy over the beam machinery; a length penalty
+    # attention decoding on the reference's encoder output of the last batch
+    prefix = whisper_prefix(cfg["tokenizer_conf"]["special_tokens"], WHISPER_INFOS["tasks"], WHISPER_INFOS["langs"])
+    eos = cfg["tokenizer_conf"]["special_tokens"]["eot"]
+    for (beam, lp), ref in zip(WHISPER_SETTINGS, gold("whisper_attention")):
         with torch.no_grad():
-            ref = attention_beam_search(model, r_out, r_mask, beam, lp, infos)
-            got = O.attention_beam_search(p, "decoder", 2, 2, r_out, r_mask, beam, prefix.tolist(), model.eos, lp, "whisper")
-        assert [list(r.tokens) for r in ref] == got, (beam, lp)
+            got = O.attention_beam_search(p, "decoder", 2, 2, r_out, r_mask, beam, prefix.tolist(), eos, lp, "whisper")
+        assert ref == got, (beam, lp)
         assert sum(len(g) for g in got) > 0

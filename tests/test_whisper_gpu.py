@@ -271,12 +271,18 @@ def test_lse_topk_sliced(M, V, k, slices):
     assert bool(same[1:].all()) and bool(same[0, 2:].all())
 
 
+NEAR_TIE = 0.15
+
+
 def test_whisper_large_widths_against_oracle():
     """The code paths only the large geometry takes - LayerNorm d = 1280, 20 heads, K = 1280 / 5120 GEMMs (128-column tiles for
     few rows, split-K residual projections), cross attention in key pieces, the sliced top-k over V = 51 866 - on a 2 + 2
     layer model of the large-v3 widths, against the CPU oracle: encoder_out vs the fp32 oracle inside the bf16 budget and
     within 3x of the bf16-emulating oracle's own distance; attention decoding (12 tokens per hypothesis, beam 4) token for
-    token against the bf16-emulating oracle run on the GPU's encoder output."""
+    token against the bf16-emulating oracle run on the GPU's encoder output.  Where the oracle's final beams end within
+    NEAR_TIE of each other they are not ordered by the arithmetic, and the bf16 path may end on either one: the emulation's
+    own 12-step score of one hypothesis moves by 0.06 between decoding utterance 1 alone and in this batch of three, where
+    its two best beams end 0.10 apart."""
     from wenet_b200.whisper import B200Whisper, whisper_prefix
     cfg = synth.recipe("whisper_wide")
     sd = synth.synth_whisper_state_dict_fast(cfg, seed=SEED, eos_beta=3.0)
@@ -306,9 +312,12 @@ def test_whisper_large_widths_against_oracle():
     res = model.decode(["attention"], xs.cuda(), xl.cuda(), beam_size=4, infos=infos)["attention"]
     prefix = whisper_prefix(cfg["tokenizer_conf"]["special_tokens"], infos["tasks"], infos["langs"])
     with torch.no_grad():
-        ref = O.attention_beam_search(sd, "decoder", 2, 20, out.cpu(), masks.cpu(), 4, prefix.tolist(), model.eos, 0.0, "whisper",
-                                      O.bf16_round, maxlen=steps + 4)
+        ref, beams = O.attention_beam_search(sd, "decoder", 2, 20, out.cpu(), masks.cpu(), 4, prefix.tolist(), model.eos, 0.0,
+                                             "whisper", O.bf16_round, maxlen=steps + 4, return_beams=True)
     got = [list(r.tokens) for r in res]
     agree = [sum(int(a == b2) for a, b2 in zip(x, y)) / max(len(y), 1) for x, y in zip(got, ref)]
-    print("whisper wide decode: GPU", got, "oracle", ref, "agreement", agree)
-    assert sum(int(x == y) for x, y in zip(got, ref)) >= 2 and min(agree) >= 0.5
+    best = [max(s for _, s in bs) for bs in beams]
+    near_tie = [any(h == g and best[b] - s <= NEAR_TIE for h, s in beams[b]) for b, g in enumerate(got)]
+    print("whisper wide decode: GPU", got, "oracle", ref, "agreement", agree, "oracle beams", beams)
+    assert sum(int(x == y) for x, y in zip(got, ref)) >= 2
+    assert all(a >= 0.5 or t for a, t in zip(agree, near_tie)), (agree, near_tie)
