@@ -405,6 +405,19 @@ int wb_op_attention(const void* q_dev, int64_t ldq, int64_t q_rows, int q_col0, 
                     const int32_t* k_len_dev, int batch, int heads, int max_q_len, int chunk_size,
                     int num_left_chunks, float scale, void* out_dev, int64_t ldo, int out_col0,
                     int v_mode, wb_stream_t stream);
+/* wb_op_attention with the modes the model paths use internally:
+ *   kbias_scaled != 0: kbias_dev already holds bias * scale * log2(e) (as wb_op_relpos_kprep's output times that factor; the
+ *     encoder's form), read by cp.async instead of being scaled in the kernel.
+ *   part_o_dev != null: split-key mode.  `batch` = blocks x splits items; item b * splits + s is piece s of the keys of query
+ *     block b (the same q_start / q_len for every piece of a block, its own k_start / k_len, possibly empty).  Scratch:
+ *     part_o_dev batch * heads * max_q_len * 64 floats, part_ml_dev batch * heads * max_q_len * 8 bytes.  A merge kernel
+ *     combines the pieces into out; a block whose pieces hold no key gets zero rows. */
+int wb_op_attention_ex(const void* q_dev, int64_t ldq, int64_t q_rows, int q_col0, const void* k_dev, int64_t ldk,
+                       int64_t k_rows, int k_col0, const void* v_dev, int64_t ldv, int64_t v_rows, int v_col0,
+                       const float* kbias_dev, int ld_kbias, const int32_t* q_start_dev, const int32_t* q_len_dev,
+                       const int32_t* k_start_dev, const int32_t* k_len_dev, int batch, int heads, int max_q_len,
+                       int chunk_size, int num_left_chunks, float scale, void* out_dev, int64_t ldo, int out_col0,
+                       int v_mode, int kbias_scaled, int splits, float* part_o_dev, void* part_ml_dev, wb_stream_t stream);
 int wb_op_relpos_kprep(const void* k_dev, int64_t ldk, const float* pos_proj_dev,
                        const int32_t* row_pos_dev, const float* bias_u_dev, const float* bias_v_dev,
                        int M, int heads, void* kprime_dev, int64_t ldkp, float* kbias_dev,
@@ -434,6 +447,34 @@ int wb_op_lse_topk(const float* logits_dev, int64_t ldl, int M, int V, int blank
  * order.  scratch_dev: M * slices * (topk * 8 + 8) + 256 bytes. */
 int wb_op_lse_topk_sliced(const float* logits_dev, int64_t ldl, int M, int V, int topk, int slices, float* topk_val_dev,
                           int32_t* topk_idx_dev, void* scratch_dev, size_t scratch_bytes, wb_stream_t stream);
+
+/* Decoder output layer of attention rescoring without the [M, N] logits.  wb_op_gemm_lse_partials writes, per row of
+ * v = A[M,K] B[N,K]^T + bias, wb_op_lse_parts(N, K) (max, sum) float pairs: one per half of each column tile, max of
+ * v * log2(e) over the half's columns and sum of 2^(v log2 e - max); a half with no column < N holds (-inf, 0).
+ * part_dev: M * wb_op_lse_parts(N, K) float pairs. */
+int wb_op_lse_parts(int N, int K);
+int wb_op_gemm_lse_partials(const void* a_dev, int64_t lda, const void* b_dev, int M, int N, int K, const float* bias_dev,
+                            float* part_dev, wb_stream_t stream);
+/* tok_logp[r] = a[s] . w[t] + bias[t] - logsumexp(row s), s = row_map[r] (identity when null), t = target[r]; the log-sum-exp
+ * comes from the partials of row s.  A target outside [0, V) gives 0 (padding positions). */
+int wb_op_lse_target_logprob(const float* part_dev, int n_parts, const void* a_dev, int64_t lda, const void* w_dev, int d,
+                             const float* bias_dev, const int32_t* target_dev, const int32_t* row_map_dev, int R, int V,
+                             float* tok_logp_dev, wb_stream_t stream);
+/* x[r] = emb[tokens[r]] * xscale + pe[pos[r]] (fp32 rows of d, d % 4 == 0) */
+int wb_op_embed_tokens(const int32_t* tokens_dev, const int32_t* pos_dev, int R, int d, const float* emb_dev,
+                       const float* pe_dev, float xscale, float* x_dev, wb_stream_t stream);
+/* score combine of attention rescoring (search.py:421-452): hypothesis h has hyp_len[h] tokens and its token log-probs at
+ * l2r[hyp_row0[h] ..] (tokens then <eos>; r2l the same for the right-to-left decoder, or null); utterance b owns
+ * hypotheses [utt_hyp0[b], + utt_nhyp[b]).  hyp_score[h] = mix of the fp32 sums + ctc_score * ctc_weight, best[b] = first
+ * maximum within the utterance (0 without hypotheses). */
+int wb_op_rescore_combine(const float* l2r_dev, const float* r2l_dev, const int32_t* hyp_row0_dev, const int32_t* hyp_len_dev,
+                          const int32_t* utt_hyp0_dev, const int32_t* utt_nhyp_dev, int batch, const double* ctc_score_dev,
+                          float ctc_weight, float reverse_weight, float* hyp_score_dev, int32_t* best_dev, wb_stream_t stream);
+/* cached self attention of one new position per decoder row (attention decoding): qkv [R][3d] bf16 of this step, d = 64 H;
+ * writes row r's K / V into slot (pos, r) of kv [L][R][2d] bf16 and ctx[r] ([R][d] bf16) = softmax(q k^T * scale) v over
+ * positions 0..pos, position j < pos read from slot (j, anc[r * anc_stride + j]). */
+int wb_op_dec_self_attn_step(const void* qkv_dev, void* kv_dev, const int32_t* anc_dev, int anc_stride, int pos, int R, int H,
+                             int d, float scale, void* ctx_dev, wb_stream_t stream);
 
 #ifdef __cplusplus
 }

@@ -102,6 +102,14 @@ _PROTOS = {
     "wb_op_logsoftmax_topk": (i32, [vp, i64, i32, i32, i32, f32, i32, vp, vp, vp]),
     "wb_op_lse_topk_sliced": (i32, [vp, i64, i32, i32, i32, i32, vp, vp, vp, sz, vp]),
     "wb_op_lse_topk": (i32, [vp, i64, i32, i32, i32, f32, i32, vp, vp, vp]),
+    "wb_op_attention_ex": (i32, [vp, i64, i64, i32, vp, i64, i64, i32, vp, i64, i64, i32, vp, i32, vp, vp,
+                                  vp, vp, i32, i32, i32, i32, i32, f32, vp, i64, i32, i32, i32, i32, vp, vp, vp]),
+    "wb_op_lse_parts": (i32, [i32, i32]),
+    "wb_op_gemm_lse_partials": (i32, [vp, i64, vp, i32, i32, i32, vp, vp, vp]),
+    "wb_op_lse_target_logprob": (i32, [vp, i32, vp, i64, vp, i32, vp, vp, vp, i32, i32, vp, vp]),
+    "wb_op_embed_tokens": (i32, [vp, vp, i32, i32, vp, vp, f32, vp, vp]),
+    "wb_op_rescore_combine": (i32, [vp, vp, vp, vp, vp, vp, i32, vp, f32, f32, vp, vp, vp]),
+    "wb_op_dec_self_attn_step": (i32, [vp, vp, vp, i32, i32, i32, i32, i32, f32, vp, vp]),
 }
 
 EXPORTED_SYMBOLS = tuple(sorted(_PROTOS))

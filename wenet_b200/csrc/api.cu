@@ -445,6 +445,24 @@ int wb_op_attention(const void* q_dev, int64_t ldq, int64_t q_rows, int q_col0, 
     a.out = out_dev; a.ldo = ldo; a.out_col0 = out_col0; a.split3_out = 0; a.v_mode = v_mode;
     return attention_forward(a, (cudaStream_t)stream);
 }
+int wb_op_attention_ex(const void* q_dev, int64_t ldq, int64_t q_rows, int q_col0, const void* k_dev, int64_t ldk,
+                       int64_t k_rows, int k_col0, const void* v_dev, int64_t ldv, int64_t v_rows, int v_col0,
+                       const float* kbias_dev, int ld_kbias, const int32_t* q_start_dev, const int32_t* q_len_dev,
+                       const int32_t* k_start_dev, const int32_t* k_len_dev, int batch, int heads, int max_q_len,
+                       int chunk_size, int num_left_chunks, float scale, void* out_dev, int64_t ldo, int out_col0,
+                       int v_mode, int kbias_scaled, int splits, float* part_o_dev, void* part_ml_dev, wb_stream_t stream) {
+    AttnArgs a;
+    a.q = q_dev; a.ldq = ldq; a.q_rows = q_rows; a.q_col0 = q_col0;
+    a.k = k_dev; a.ldk = ldk; a.k_rows = k_rows; a.k_col0 = k_col0;
+    a.v = v_dev; a.ldv = ldv; a.v_rows = v_rows; a.v_col0 = v_col0;
+    a.kbias = kbias_dev; a.ld_kbias = ld_kbias; a.kbias_scaled = kbias_scaled;
+    a.q_start = q_start_dev; a.q_len = q_len_dev; a.k_start = k_start_dev; a.k_len = k_len_dev;
+    a.batch = batch; a.heads = heads; a.max_q_len = max_q_len;
+    a.chunk_size = chunk_size; a.num_left_chunks = num_left_chunks; a.scale = scale;
+    a.out = out_dev; a.ldo = ldo; a.out_col0 = out_col0; a.split3_out = 0; a.v_mode = v_mode;
+    a.part_o = part_o_dev; a.part_ml = part_ml_dev; a.splits = splits;
+    return attention_forward(a, (cudaStream_t)stream);
+}
 int wb_op_relpos_kprep(const void* k_dev, int64_t ldk, const float* pos_proj_dev, const int32_t* row_pos_dev,
                        const float* bias_u_dev, const float* bias_v_dev, int M, int heads, void* kprime_dev,
                        int64_t ldkp, float* kbias_dev, wb_stream_t stream) {
@@ -479,6 +497,39 @@ int wb_op_lse_topk_sliced(const float* logits_dev, int64_t ldl, int M, int V, in
     WB_REQUIRE(scratch_bytes >= lse_topk_sliced_scratch_bytes(M, slices, topk), WB_ERR_WORKSPACE, "lse_topk_sliced: scratch %zu < %zu",
                scratch_bytes, lse_topk_sliced_scratch_bytes(M, slices, topk));
     return lse_topk_sliced(logits_dev, ldl, M, V, topk, slices, topk_val_dev, topk_idx_dev, scratch_dev, (cudaStream_t)stream);
+}
+
+int wb_op_lse_parts(int N, int K) { return lse_parts(N, K); }
+int wb_op_gemm_lse_partials(const void* a_dev, int64_t lda, const void* b_dev, int M, int N, int K, const float* bias_dev,
+                            float* part_dev, wb_stream_t stream) {
+    return gemm_lse_partials(a_dev, lda, nullptr, b_dev, M, N, K, bias_dev, reinterpret_cast<float2*>(part_dev),
+                             (cudaStream_t)stream);
+}
+int wb_op_lse_target_logprob(const float* part_dev, int n_parts, const void* a_dev, int64_t lda, const void* w_dev, int d,
+                             const float* bias_dev, const int32_t* target_dev, const int32_t* row_map_dev, int R, int V,
+                             float* tok_logp_dev, wb_stream_t stream) {
+    return lse_target_logprob(reinterpret_cast<const float2*>(part_dev), n_parts, a_dev, lda, w_dev, d, bias_dev, target_dev,
+                              row_map_dev, R, V, tok_logp_dev, (cudaStream_t)stream);
+}
+int wb_op_embed_tokens(const int32_t* tokens_dev, const int32_t* pos_dev, int R, int d, const float* emb_dev,
+                       const float* pe_dev, float xscale, float* x_dev, wb_stream_t stream) {
+    return embed_tokens(tokens_dev, pos_dev, R, d, emb_dev, pe_dev, xscale, x_dev, (cudaStream_t)stream);
+}
+int wb_op_rescore_combine(const float* l2r_dev, const float* r2l_dev, const int32_t* hyp_row0_dev, const int32_t* hyp_len_dev,
+                          const int32_t* utt_hyp0_dev, const int32_t* utt_nhyp_dev, int batch, const double* ctc_score_dev,
+                          float ctc_weight, float reverse_weight, float* hyp_score_dev, int32_t* best_dev, wb_stream_t stream) {
+    RescoreArgs a;
+    a.l2r = l2r_dev; a.r2l = r2l_dev;
+    a.hyp_row0 = hyp_row0_dev; a.hyp_len = hyp_len_dev;
+    a.utt_hyp0 = utt_hyp0_dev; a.utt_nhyp = utt_nhyp_dev; a.batch = batch;
+    a.ctc_score = ctc_score_dev;
+    a.ctc_weight = ctc_weight; a.reverse_weight = reverse_weight;
+    a.hyp_score = hyp_score_dev; a.best = best_dev;
+    return rescore_combine(a, (cudaStream_t)stream);
+}
+int wb_op_dec_self_attn_step(const void* qkv_dev, void* kv_dev, const int32_t* anc_dev, int anc_stride, int pos, int R, int H,
+                             int d, float scale, void* ctx_dev, wb_stream_t stream) {
+    return dec_self_attn_step(qkv_dev, kv_dev, anc_dev, anc_stride, pos, R, H, d, scale, ctx_dev, (cudaStream_t)stream);
 }
 
 // ---------------------------------------------------------------- Whisper log-mel

@@ -312,6 +312,27 @@ int attention_beam_step_op(const float* topv, const int* topi, const float* scor
     return WB_OK;
 }
 
+// the self-attention step kernel keeps one score + one slot per past position and warp in shared memory
+constexpr size_t kSaSmemMax = 200 * 1024;
+
+int dec_self_attn_step(const void* qkv, void* kv, const int* anc, int anc_stride, int pos, int R, int H, int d, float scale,
+                       void* ctx, cudaStream_t st) {
+    if (R <= 0) return WB_OK;
+    WB_REQUIRE(pos >= 0 && H >= 1 && d == H * 64 && (pos == 0 || anc_stride >= pos), WB_ERR_BAD_ARG,
+               "dec_self_attn_step: bad argument (pos %d, H %d, d %d, anc_stride %d)", pos, H, d, anc_stride);
+    const size_t smem = (size_t)SA_WARPS * 2 * (pos + 1) * sizeof(float);
+    WB_REQUIRE(smem <= kSaSmemMax, WB_ERR_UNSUPPORTED, "dec_self_attn_step: position %d exceeds the %zu positions the kernel holds",
+               pos, kSaSmemMax / (SA_WARPS * 2 * sizeof(float)));
+    WB_SET_MAX_DYN_SMEM(dec_self_attn_step_kernel, kSaSmemMax);
+    ProfScope _ps(PT_ATTENTION, st, 0.0);
+    WB_CHECK_CUDA(launch_maybe_pdl(dec_self_attn_step_kernel, dim3(ceil_div(R * H, SA_WARPS)), dim3(SA_WARPS * 32), smem, st,
+                                   reinterpret_cast<const __nv_bfloat16*>(qkv), reinterpret_cast<__nv_bfloat16*>(kv), anc,
+                                   anc_stride, pos, R, H, d, scale, reinterpret_cast<__nv_bfloat16*>(ctx)));
+    count_launch();
+    WB_CHECK_LAUNCH();
+    return WB_OK;
+}
+
 size_t attention_beam_workspace_bytes(const Model* m, long long enc_rows, int batch, int beam, int max_len) {
     AbPlan P;
     ab_layout(m, enc_rows, batch, beam, max_len, &P);
@@ -435,12 +456,9 @@ int attention_beam_search(const Model* m, const void* enc_bf16, long long enc_ro
     int pos = 0;
     std::vector<int> ended_host(batch, 0);
     int steps = 0;
-    // the self-attention step kernel keeps one score + one slot per past position and warp in shared memory
-    constexpr size_t kSaSmemMax = 200 * 1024;
     WB_REQUIRE((size_t)SA_WARPS * 2 * max_len * sizeof(float) <= kSaSmemMax, WB_ERR_UNSUPPORTED,
                "attention_beam_search: max_len %d exceeds the %zu positions the self-attention step kernel holds", max_len,
                kSaSmemMax / (SA_WARPS * 2 * sizeof(float)));
-    WB_SET_MAX_DYN_SMEM(dec_self_attn_step_kernel, kSaSmemMax);
     PdlScope pdl_scope;   // the step loop is a chain of short dependent launches: GEMMs start ahead of their predecessor's end
     // token positions 0 .. max_len - 2 are consumed; the step at position `pos` produces the token of position pos + 1
     for (pos = 0; pos + 1 < max_len; ++pos) {
@@ -452,14 +470,7 @@ int attention_beam_search(const Model* m, const void* enc_bf16, long long enc_ro
             const DecLayer& Ly = D.layers[li];
             __nv_bfloat16* kvl = reinterpret_cast<__nv_bfloat16*>(ws + P.o_kv) + (size_t)li * L * R * 2 * d;
             RC(gemm_bf16(a, d, &Ly.sa_qkv.tmap, Ly.sa_qkv.w, R, 3 * d, d, Ly.sa_qkv.b, EPI_BF16, 1.0f, qkv, 3 * d, 0, st));
-            {
-                ProfScope _ps(PT_ATTENTION, st, 0.0);
-                const size_t smem = (size_t)SA_WARPS * 2 * (pos + 1) * sizeof(float);
-                WB_CHECK_CUDA(launch_maybe_pdl(dec_self_attn_step_kernel, dim3(ceil_div(R * H, SA_WARPS)), dim3(SA_WARPS * 32), smem,
-                                               st, qkv, kvl, anc[cur], L, pos, R, H, d, scale, ctx));
-                count_launch();
-                WB_CHECK_LAUNCH();
-            }
+            RC(dec_self_attn_step(qkv, kvl, anc[cur], L, pos, R, H, d, scale, ctx, st));
             RC(resid_then_norm(ctx, d, Ly.sa_out, R, d, x, Ly.n2, c.dec_ln_eps, a, st));
             RC(gemm_bf16(a, d, &Ly.ca_q.tmap, Ly.ca_q.w, R, d, d, Ly.ca_q.b, EPI_BF16, 1.0f, q, d, 0, st));
             {

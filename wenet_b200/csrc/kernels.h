@@ -144,7 +144,8 @@ struct AttnArgs {
     // split-key mode (flash-decoding): `batch` = blocks x splits items, item b * splits + s holding piece s of the keys of
     // query block b (same q_start / q_len for the pieces of a block, its own k_start / k_len); the kernel leaves
     // unnormalised fp32 partial outputs part_o [batch][heads][max_q_len][64] and (reference point, sum) part_ml
-    // [batch][heads][max_q_len] (float2), and a merge kernel writes `out`.  max_q_len <= 128.
+    // [batch][heads][max_q_len] (float2), and a merge kernel writes `out`.  Any max_q_len (blocks of more than 128 queries
+    // take several CTAs per piece, each writing its own rows of the part buffers).
     float* part_o = nullptr;
     void* part_ml = nullptr;
     int splits = 1;

@@ -99,6 +99,12 @@ int attention_beam_search(const Model* m, const void* enc_bf16, long long enc_ro
                           int max_len, float length_penalty, int32_t* out_tokens_dev, int out_stride, int32_t* out_lens_dev,
                           float* out_scores_dev, int32_t* steps_run_host, void* ws, size_t ws_bytes, cudaStream_t st);
 
+// cached self attention of ONE new position per row (R = batch x beam rows, H heads of 64, d = 64 H): qkv [R][3d] bf16 of this
+// step; writes K / V of row r into cache slot kv[pos][r] ([L][R][2d] bf16) and ctx[r] (bf16 [R][d]) = softmax attention over
+// positions 0..pos of r's history, position j < pos read from slot (j, anc[r * anc_stride + j])
+int dec_self_attn_step(const void* qkv, void* kv, const int* anc, int anc_stride, int pos, int R, int H, int d, float scale,
+                       void* ctx, cudaStream_t st);
+
 int attention_beam_step_op(const float* topv, const int* topi, const float* score_in, const int* end_in, const int* hyp_in,
                            const int* anc_in, int batch, int beam, int L, int pos, int eos, float* score_out, int* end_out,
                            int* hyp_out, int* anc_out, int* cur_tok, int* cur_pos, int* utt_ended, cudaStream_t st);
